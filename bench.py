@@ -24,6 +24,9 @@ N > 1) -> argmax.
   next  : chooser.next() wall-ms through the plugin API at the SAME workload, steady state (no burn-in), with the phase
           split (MCMC / grid pass 1 / L-BFGS refinement / grid pass 2) and the CPU port's time as counts x unit times.
   --impl reference : the CPU implementation as its own arm (rank 0 only).
+  --dump-outputs DIR : after the timed steps, what the last step of each EI leg returned: ei_sum (M,) and argmax of the
+          value leg, ei_matrix_e2e (M, S) and argmax_e2e of the e2e leg.  The inputs are seeded, so two builds run with
+          the same arguments can be compared output for output.
 
 Multi-GPU: hyper-samples are sharded round-robin over ranks (total work fixed -> "scaling": "strong"); the
 only exchange is one NCCL all-reduce of M floats.
@@ -304,7 +307,7 @@ def run_b200_arm(args, D, N, M, S):
             ei_sum = torch.zeros((ldm,), dtype=torch.float64, device=eng.device)
         parallel.allreduce_sum_(ei_sum)
         idx, _ = eng.topk(ei_sum, M, 1)
-        return idx
+        return ei_sum, idx
 
     # ---- e2e leg: the plugin call.  GPEIOptChooserB200.ei_over_hypers is the drop-in for OPT:331-341; the per-second
     # plugin's method reproduces the reference's column-0-only early return (PSEC:302), so that workload goes through the
@@ -364,8 +367,10 @@ def run_b200_arm(args, D, N, M, S):
         step_resident()
     eng.check_deferred()
     sampler.mark_begin()
-    ms, _, launches, stages, idx = timed(step_resident, args.steps, with_timers=True)
+    ms, _, launches, stages, (ei_sum, idx) = timed(step_resident, args.steps, with_timers=True)
     eng.check_deferred()
+    if args.dump_outputs and rank == 0:       # copied now: the e2e leg below may reuse the engine's buffers
+        dump = {"ei_sum": ei_sum[:M].double().cpu().numpy(), "argmax": np.array([float(idx.cpu()[0])])}
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = ms / args.steps
     value = M / (ms_per_step * 1e-3)
@@ -380,6 +385,9 @@ def run_b200_arm(args, D, N, M, S):
     step_e2e()
     _, wall_ms, _, _, (ei_host, best_idx) = timed(step_e2e, args.steps)
     e2e_ms = wall_ms / args.steps
+    if args.dump_outputs and rank == 0:
+        dump.update(ei_matrix_e2e=ei_host, argmax_e2e=np.array([float(best_idx)]))
+        dump_outputs(args.dump_outputs, dump)
     esz = 4
     n_gp = 2 if per_s else 1
     h2d = esz * (comp.size + cand.size + n_gp * vals.size) + esz * n_gp * Sl * (D + 3)
@@ -449,6 +457,23 @@ def run_b200_arm(args, D, N, M, S):
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64 * 10 ** 6 - 4096          # 64 MB, less room for the .npy headers
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as path/<name>.npy in float64.  When the EI matrix would take the total past DUMP_BYTES, a fixed
+    seeded sample of its rows is written instead, with the row indices as ei_matrix_e2e_rows."""
+    os.makedirs(path, exist_ok=True)
+    mat = arrays["ei_matrix_e2e"]
+    room = DUMP_BYTES - sum(a.nbytes for k, a in arrays.items() if k != "ei_matrix_e2e")
+    if mat.nbytes > room:
+        keep = room // (8 * (mat.shape[1] + 1)) - 1                  # float64 rows plus their float64 indices
+        rows = np.sort(np.random.RandomState(0).choice(mat.shape[0], keep, replace=False))
+        arrays = dict(arrays, ei_matrix_e2e=mat[rows], ei_matrix_e2e_rows=rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def next_wall_ms(args, D, N, M, S, backend):
     """Second half of BASELINE.json's metric: chooser.next() wall-ms through the plugin API at the benched workload
     (MCMC chain with the GPU float64 log-likelihood -> grid pass -> L-BFGS refinement with cached factors -> grid pass),
@@ -506,7 +531,13 @@ def main():
     ap.add_argument("--no-next", action="store_true", help="skip the chooser.next() wall-ms leg")
     ap.add_argument("--next-calls", type=int, default=1, help="timed next() calls")
     ap.add_argument("--next-cpu", action="store_true", help="also run the CPU port of next() for real (slow)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results of both EI legs to DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     D, N, M, S = WORKLOADS[args.workload]
     if args.samples:
         S = args.samples

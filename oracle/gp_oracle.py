@@ -8,8 +8,8 @@ Pinning: the reference ships no tests or golden vectors (SURVEY.md section 4), s
 pinned against the reference ITSELF, executed in the build container through
 ``oracle/ref_shim.py``: ``tests/golden/make_golden.py`` froze the reference's outputs into
 ``tests/golden/*.npz`` and ``tests/test_oracle_golden.py`` checks every function here against
-them (rtol 1e-9 or tighter); ``tests/test_oracle_vs_reference.py`` re-checks directly against
-the live reference whenever ``/root/reference`` exists.
+them (rtol 1e-9 or tighter); ``tests/test_oracle_vs_reference.py`` re-checks against the
+reference's outputs on a second set of seeded inputs (``tests/golden/make_golden_live.py``).
 
 Reference files restated (paths relative to ``/root/reference/spearmint/spearmint``):
   GP   = gp.py                          OPT  = chooser/GPEIOptChooser.py

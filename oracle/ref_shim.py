@@ -4,13 +4,12 @@ Nothing is copied: the Python-2 files under ``/root/reference`` are read at run 
 passed through a handful of mechanical py2->py3 regex rewrites (SURVEY.md section 8(c)) and
 ``exec``-ed into fresh module objects.  It exists so that
 
-  * ``tests/golden/make_golden.py`` can freeze golden input/output vectors of the real
-    reference (``gp.py``, ``GPEIOptChooser.py``, ``GPEIperSecChooser.py``, ``GPEIChooser.py``),
-  * ``tests/test_oracle_vs_reference.py`` can pin ``oracle/gp_oracle.py`` (the numpy
-    restatement) directly against the reference whenever ``/root/reference`` is present.
+  * ``tests/golden/make_golden*.py`` can freeze golden input/output vectors of the real
+    reference (``gp.py``, ``GPEIOptChooser.py``, ``GPEIperSecChooser.py``, ``GPEIChooser.py``,
+    the spearmint-lite controller).
 
-``/root/reference`` does not exist on the GPU box, so nothing imported by ``-m gpu`` tests,
-``__graft_entry__.smoke()`` or ``bench.py`` may depend on this file at run time.
+The reference tree is not part of this repository, so no test, ``__graft_entry__.smoke()``
+or ``bench.py`` may depend on this file at run time.
 The product package ``spearmint_b200`` never imports anything from ``oracle/``.
 """
 import os

@@ -1,19 +1,17 @@
-"""CPU, build container only (needs /root/reference): BASELINE config 1 -- the reference's UNMODIFIED spearmint-lite
-controller proposes Branin experiments through our chooser, loaded by name via the 3-line stub of INTEGRATION.md.
-The controller, GridMap, results.dat parsing and candidate generation are the reference's own code (py3 shim);
-only the numerics behind the chooser are the oracle stand-in here (no GPU in this container) -- the same chooser
-class is exercised with the real DeviceBackend in tests/test_gpu_chooser.py."""
+"""CPU: BASELINE config 1 -- the reference's UNMODIFIED spearmint-lite controller proposing Branin experiments through our
+chooser, loaded by name via the 3-line stub of INTEGRATION.md.  tests/golden/lite_branin.npz records every
+chooser.next() call that controller made in such a run (tests/golden/make_golden_live.py) and what the chooser returned;
+this test imports the chooser the way the controller does ('chooser.' + name), makes a fresh one per proposal as the
+controller does, and replays those calls.  Only the numerics behind the chooser are the oracle stand-in here (no GPU
+needed) -- the same chooser class is exercised with the real DeviceBackend in tests/test_gpu_chooser.py."""
+import importlib
 import os
-import shutil
 import sys
-import types
 
 import numpy as np
-import pytest
 
-from oracle import ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+from tests.helpers import load
+from tests.oracle_backend import OracleBackend
 
 STUB = "from spearmint_b200.chooser.GPEIOptChooserB200 import *  # noqa: F401,F403\n"
 
@@ -26,38 +24,43 @@ def branin(x):
 
 
 def test_spearmint_lite_drives_the_dropin_chooser(tmp_path, monkeypatch):
-    lite = ref_shim.load_lite()
+    g = load("lite_branin")
     # the stub a maintainer drops into spearmint/spearmint/chooser/
-    plug = tmp_path / "plugins"
-    plug.mkdir()
+    plug = tmp_path / "plugins" / "chooser"
+    plug.mkdir(parents=True)
+    (plug / "__init__.py").write_text("")
     (plug / "GPEIOptChooserB200.py").write_text(STUB)
-    sys.modules["chooser"].__path__ = [str(plug)]
-    sys.modules.pop("chooser.GPEIOptChooserB200", None)
-    # numerics: oracle stand-in (CPU container); the product default is DeviceBackend and raises without CUDA
+    monkeypatch.syspath_prepend(str(tmp_path / "plugins"))
+    for name in [m for m in sys.modules if m == "chooser" or m.startswith("chooser.")]:
+        monkeypatch.delitem(sys.modules, name)
+    module = importlib.import_module("chooser.GPEIOptChooserB200")
+    # numerics: oracle stand-in; the product default is DeviceBackend and raises without CUDA
     import spearmint_b200.backend as be
-    from tests.oracle_backend import OracleBackend
     monkeypatch.setattr(be, "DeviceBackend", lambda **kw: OracleBackend())
 
     expt = tmp_path / "braninpy"
     expt.mkdir()
-    shutil.copy(os.path.join(ref_shim.REF_ROOT, "spearmint-lite", "braninpy", "config.json"), str(expt))
-    opts = types.SimpleNamespace(num_jobs=1, max_finished_jobs=1000, chooser_module="GPEIOptChooserB200",
-                                 chooser_args="mcmc_iters=3,burnin=5,grid_subset=4,use_multiprocessing=0",
-                                 grid_size=300, grid_seed=1, config_file="config.json", results_file="results.dat")
-    res = expt / "results.dat"
-    np.random.seed(0)
+    lines = str(g["results_dat"]).splitlines()          # the controller's results.dat after the run (values filled in)
+    assert len(lines) == int(g["iters"]) == 8
+    np.random.seed(int(g["seed"]))
     best = np.inf
-    for it in range(8):
-        lite.main_controller(opts, [str(expt)])            # appends one "P P x1 x2" line (LITE:199-215)
-        lines = res.read_text().splitlines()
-        assert lines[-1].startswith("P P ")
-        x = [float(t) for t in lines[-1].split()[2:]]
-        assert len(x) == 2 and all(0.0 <= t <= 1.0 for t in x)
-        y = branin(x)
-        best = min(best, y)
-        lines[-1] = "%f 1 %s" % (y, " ".join(lines[-1].split()[2:]))      # braninrunner.py fills the result in
-        res.write_text("\n".join(lines) + "\n")
-    assert len(res.read_text().splitlines()) == 8
+    for i in range(int(g["iters"])):
+        c = {k: g["%s_%d" % (k, i)] for k in ("grid", "values", "durations", "candidates", "pending", "complete",
+                                              "ret_tuple", "ret_index", "ret_point")}
+        # the controller passes a float, not an array, when exactly one result is complete
+        durations = float(c["durations"]) if c["durations"].ndim == 0 else c["durations"]
+        ch = module.init(str(expt), str(g["chooser_args"]))
+        ret = ch.next(c["grid"], c["values"], durations, c["candidates"], c["pending"], c["complete"])
+        if bool(c["ret_tuple"]):
+            assert isinstance(ret, tuple) and ret[0] == int(c["ret_index"])
+            x = np.asarray(ret[1], dtype=float)
+            np.testing.assert_allclose(x, c["ret_point"], rtol=0, atol=1e-6)
+        else:
+            assert int(ret) == int(c["ret_index"])
+            x = c["grid"][int(ret)]
+        assert x.shape == (2,) and np.all((0.0 <= x) & (x <= 1.0))
+        np.testing.assert_allclose(x, [float(t) for t in lines[i].split()[2:]], rtol=0, atol=1e-6)   # what it wrote
+        best = min(best, branin(x))
     # GP-EI picked the last 6 (the first two proposals are "candidates[0]" with < 2 completed, OPT:221-222)
     assert os.path.exists(str(expt / "spearmint_b200.chooser.GPEIOptChooserB200.pkl"))
     assert best < 25.0      # Branin over the unit square spans 0.4 .. 300; 8 evaluations already land in the basin

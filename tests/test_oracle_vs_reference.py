@@ -1,66 +1,38 @@
-"""The oracle against the LIVE reference (executed through oracle/ref_shim.py) -- runs wherever /root/reference exists
-(the build container), skipped on the GPU box.  The committed golden fixtures (tests/golden/*.npz, test_oracle_golden.py)
-pin the same functions on frozen outputs; this file re-checks them on fresh random inputs."""
+"""The oracle against the reference on seeded random problems other than those of test_oracle_golden.py: the reference's
+outputs, and the exact inputs it was given, are frozen in tests/golden/oracle_vs_ref.npz
+(tests/golden/make_golden_live.py executes the reference through oracle/ref_shim.py to produce them)."""
 import numpy as np
 import pytest
 
 from oracle import gp_oracle as O
-from oracle import ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+from tests.helpers import load
 
 
 @pytest.fixture(scope="module")
-def R():
-    return ref_shim.load()
-
-
-def _problem(seed, D=3, N=25, M=40):
-    rs = np.random.RandomState(seed)
-    comp, cand = rs.rand(N, D), rs.rand(M, D)
-    y = np.sin(3 * comp).sum(1) + 0.05 * rs.randn(N)
-    return comp, cand, (y - y.mean()) / y.std(), rs
+def g():
+    return load("oracle_vs_ref")
 
 
 @pytest.mark.parametrize("kind", ["SE", "ARDSE", "Matern32", "Matern52"])
-def test_kernels_and_logprob(R, kind):
-    gp = R["gp"]
-    comp, cand, vals, rs = _problem(1)
-    ls = rs.uniform(0.4, 1.8, comp.shape[1])
-    f = getattr(gp, kind)
-    np.testing.assert_allclose(O.kernel(kind, ls, comp), f(ls, comp), rtol=1e-12, atol=1e-14)
-    np.testing.assert_allclose(O.kernel(kind, ls, comp, cand), f(ls, comp, cand), rtol=1e-12, atol=1e-14)
-    g = gp.GP(kind)
-    g.real_init(comp.shape[1], vals)
-    g.ls, g.amp2, g.noise, g.mean = ls, 1.3, 2e-3, 0.1
-    np.testing.assert_allclose(O.gp_logprob(kind, 0.1, 2e-3, 1.3, ls, comp, vals), g.logprob(comp, vals), rtol=1e-11)
+def test_kernels_and_logprob(g, kind):
+    comp, cand, vals, ls = (g["k_%s_%s" % (kind, k)] for k in ("comp", "cand", "vals", "ls"))
+    np.testing.assert_allclose(O.kernel(kind, ls, comp), g["k_%s_self" % kind], rtol=1e-12, atol=1e-14)
+    np.testing.assert_allclose(O.kernel(kind, ls, comp, cand), g["k_%s_cross" % kind], rtol=1e-12, atol=1e-14)
+    np.testing.assert_allclose(O.gp_logprob(kind, 0.1, 2e-3, 1.3, ls, comp, vals), g["k_%s_logprob" % kind], rtol=1e-11)
 
 
-def test_compute_ei_with_and_without_pending(R, tmp_path):
-    OPT = R["OPT"]
-    comp, cand, vals, rs = _problem(2)
-    ch = OPT.init(str(tmp_path), "mcmc_iters=2,burnin=1,use_multiprocessing=0")
-    ch.D = comp.shape[1]
-    ch.randomstate = np.random.get_state()
-    ch.mean, ch.noise, ch.amp2, ch.ls = 0.05, 1e-3, 0.9, rs.uniform(0.4, 1.8, ch.D)
-    h = (ch.mean, ch.noise, ch.amp2, ch.ls)
-    np.testing.assert_allclose(O.compute_ei("Matern52", h, comp, np.zeros((0, ch.D)), cand, vals),
-                               ch.compute_ei(comp, np.zeros((0, ch.D)), cand, vals), rtol=1e-9, atol=1e-14)
-    pend = rs.rand(2, ch.D)
-    np.random.set_state(ch.randomstate)
-    normals = np.random.randn(2, ch.pending_samples)
-    np.testing.assert_allclose(O.compute_ei("Matern52", h, comp, pend, cand, vals, normals),
-                               ch.compute_ei(comp, pend, cand, vals), rtol=1e-9, atol=1e-14)
+def test_compute_ei_with_and_without_pending(g):
+    comp, cand, vals = g["ei_comp"], g["ei_cand"], g["ei_vals"]
+    h = (float(g["ei_mean"]), float(g["ei_noise"]), float(g["ei_amp2"]), g["ei_ls"])
+    np.testing.assert_allclose(O.compute_ei("Matern52", h, comp, np.zeros((0, comp.shape[1])), cand, vals),
+                               g["ei_nopend"], rtol=1e-9, atol=1e-14)
+    np.testing.assert_allclose(O.compute_ei("Matern52", h, comp, g["ei_pend"], cand, vals, g["ei_normals"]),
+                               g["ei_withpend"], rtol=1e-9, atol=1e-14)
 
 
-def test_sobol_and_optimize_hypers(R):
+def test_sobol_and_optimize_hypers(g):
     from oracle import sobol_oracle as SO
-    sb, gp = R["sobol_lib"], R["gp"]
-    assert np.array_equal(SO.i4_sobol_generate(6, 50, 2), sb.i4_sobol_generate(6, 50, 2))
-    comp, cand, vals, rs = _problem(3, D=2, N=20)
-    g = gp.GP("Matern52")
-    g.real_init(2, vals)
-    g.optimize_hypers(comp, vals)
-    m, noise, amp2, ls = O.gp_optimize_hypers("Matern52", comp, vals)
-    np.testing.assert_allclose([m, noise, amp2], [g.mean, g.noise, g.amp2], rtol=1e-6)
-    np.testing.assert_allclose(ls, g.ls, rtol=1e-6)
+    assert np.array_equal(SO.i4_sobol_generate(6, 50, 2), g["sobol_6x50_skip2"])
+    m, noise, amp2, ls = O.gp_optimize_hypers("Matern52", g["mll_comp"], g["mll_vals"])
+    np.testing.assert_allclose([m, noise, amp2], [g["mll_mean"], g["mll_noise"], g["mll_amp2"]], rtol=1e-6)
+    np.testing.assert_allclose(ls, g["mll_ls"], rtol=1e-6)
